@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # product arm
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path on this box's host cores
+    python bench.py ... --dump-outputs DIR                   # also write what the timed steps computed (dump_outputs)
 
 One STEP = one pass of the hot path over one batch of synthetic events: ingest_kernel (count-min / HLL / process histograms; a
 response sample of a hot service updates its dense row of value bins, any other becomes a sort key), 4 one-sweep radix passes,
@@ -64,7 +65,12 @@ def parse():
     ap.add_argument("--cpu-sample", type=int, default=20_000_000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the engine's answers (a fixed sample, see dump_outputs) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 def rank_service_ids(rank):
@@ -72,6 +78,11 @@ def rank_service_ids(rank):
     ids = synth.splitmix64(np.arange(1, NSVC + 1, dtype=np.uint64) + np.uint64(rank * NSVC))
     ids[ids == 0] = 1
     return ids
+
+
+def rank_task_ids(rank):
+    from gyeeta_b200 import synth
+    return synth.splitmix64(np.arange(1, NTASK + 1, dtype=np.uint64) + np.uint64((1 << 40) + rank * NTASK))
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -83,7 +94,7 @@ def gen_events_gpu(torch, n, seed, rank, world, dev):
     g.manual_seed(seed)
     # a service id is unique per host (CityHash of host + netns + ip + port in the reference): every rank owns its own ids
     svc_ids = torch.from_numpy(rank_service_ids(rank).view(np.int64)).to(dev)
-    task_ids = torch.from_numpy(synth.splitmix64(np.arange(1, NTASK + 1, dtype=np.uint64) + np.uint64((1 << 40) + rank * NTASK)).view(np.int64)).to(dev)
+    task_ids = torch.from_numpy(rank_task_ids(rank).view(np.int64)).to(dev)
     cdf_s = torch.from_numpy(synth.zipf_cdf(NSVC, ZIPF_S)).to(dev)
     cdf_t = torch.from_numpy(synth.zipf_cdf(NTASK, ZIPF_S)).to(dev)
     out = torch.empty((n, 4), dtype=torch.int64, device=dev)
@@ -440,6 +451,70 @@ def run_reference(args):
 
 
 # ---------------------------------------------------------------------------------------------------------------
+# outputs of the timed path
+# ---------------------------------------------------------------------------------------------------------------
+DUMP_SEED = 20261017
+DUMP_SVCS = 2048            # the 64 hottest services + a seeded sample of the rest
+DUMP_TASKS = 1024
+DUMP_HLL_SVCS = 256
+DUMP_CMS_CELLS = 1 << 20
+
+
+def dump_outputs(eng, ge, rank, world, out_dir):
+    """What a caller reads back after the timed steps, from a fixed seeded sample of the state (~39 MB): for DUMP_SVCS of this
+    rank's services the response histogram of the open window (hist_resp: count, sum per bucket; hist_resp_total_max), every
+    numeric field of the query_svcs summary (summary_<field>), the t-digest centroids (zero-padded to TD_CAP) and for the first
+    DUMP_HLL_SVCS of them the HLL registers; the three process histograms of DUMP_TASKS tasks; DUMP_CMS_CELLS count-min cells
+    (count and kbytes halves) and the engine's event counters. Ids are given as indices into rank_service_ids / rank_task_ids.
+    Everything is float64 (integers below 2^53, exact) except the HLL registers (float32). With world > 1 each rank writes
+    its own files, suffixed _rank<r>."""
+    rng = np.random.default_rng(DUMP_SEED)
+    svc_idx = np.union1d(np.arange(64), rng.choice(np.arange(64, NSVC), DUMP_SVCS - 64, replace=False))
+    task_idx = np.sort(rng.choice(NTASK, DUMP_TASKS, replace=False))
+    cells = np.sort(rng.choice(eng.cfg.cms_depth << eng.cfg.cms_log2_width, DUMP_CMS_CELLS, replace=False))
+    svc_ids, task_ids = rank_service_ids(rank)[svc_idx], rank_task_ids(rank)[task_idx]
+    out = {"svc_index": svc_idx, "task_index": task_idx, "cms_cell": cells}
+
+    hist = np.zeros((len(svc_ids), 15, 2)); tot_max = np.zeros((len(svc_ids), 2))
+    td_means = np.zeros((len(svc_ids), ge.TD_CAP)); td_weights = np.zeros((len(svc_ids), ge.TD_CAP)); td_min_max = np.zeros((len(svc_ids), 2))
+    for i, sid in enumerate(svc_ids):
+        h = eng.export_hist(int(sid), ge.HIST_RESP_CUR)
+        if h is not None:
+            hist[i, :, 0], hist[i, :, 1], tot_max[i] = h[0]["count"], h[0]["sum"], h[1:]
+        t = eng.export_tdigest(int(sid))
+        if t is not None:
+            td_means[i, : len(t[0])], td_weights[i, : len(t[1])], td_min_max[i] = t[0], t[1], t[2:]
+    out.update(hist_resp=hist, hist_resp_total_max=tot_max, tdigest_means=td_means, tdigest_weights=td_weights, tdigest_min_max=td_min_max)
+    summ = eng.query_svcs(svc_ids)
+    for f, _ in ge.SvcSummary._fields_:
+        if f != "glob_id":
+            out["summary_" + f] = np.array([s[f] for s in summ], dtype=np.float64)
+    hll = np.zeros((DUMP_HLL_SVCS, 1 << eng.cfg.hll_p), dtype=np.float32)
+    for i, sid in enumerate(svc_ids[:DUMP_HLL_SVCS]):
+        r = eng.export_hll(int(sid))
+        if r is not None:
+            hll[i] = r
+    out["hll_registers"] = hll
+
+    th = np.zeros((len(task_ids), 3, 15, 2))
+    for i, tid in enumerate(task_ids):
+        for j, which in enumerate((ge.HIST_TASK_CPU_PCT, ge.HIST_TASK_CPU_DELAY, ge.HIST_TASK_BLKIO_DELAY)):
+            h = eng.export_hist(int(tid), which)
+            if h is not None:
+                th[i, j, :, 0], th[i, j, :, 1] = h[0]["count"], h[0]["sum"]
+    out["hist_task"] = th
+    cms = eng.export_cms()[cells]
+    out["cms_count"], out["cms_kbytes"] = cms & np.uint64(0xFFFFFFFF), cms >> np.uint64(32)
+    st = eng.stats()
+    out["counters"] = np.array([st[k] for k in ("events_in", "events_dropped", "events_resp", "events_tcp", "events_task", "nsvcs", "ntasks")])
+
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
+# ---------------------------------------------------------------------------------------------------------------
 # product arm
 # ---------------------------------------------------------------------------------------------------------------
 def main():
@@ -533,6 +608,8 @@ def main():
     dev_ms = t0.elapsed_time(t1)
     launches = eng.stats()["kernel_launches"] - launches0           # kernels of libgysketch.so launched inside the timed region
     ms_ing, ms_td, nb = eng.profile_read()
+    if args.dump_outputs:
+        dump_outputs(eng, ge, rank, world, args.dump_outputs)       # before the diagnostic batches below change the state
     # share of the events that took the hot-row way (two REDs into the service's dense value bins inside ingest_kernel instead of a
     # sort key): read from the engine after the timed region — response samples of the last batch minus its sort keys
     resp0 = eng.stats()["events_resp"]

@@ -1,12 +1,12 @@
 """Pins the CPU oracle (oracle/gysk_oracle.c) before anything trusts it:
   1. the reference's own asserted fixture, test/test_histogram.cc:29-147 (bucket ids + 4 percentiles);
   2. golden vectors produced by RUNNING the reference here (tests/golden/*.npz, made by make_golden.py);
-  3. live comparison with the compiled reference (oracle/_ref/libgyref.so) on random streams, when present.
+  3. outputs of the compiled reference (oracle/_ref/libgyref.so) on random streams, recorded in tests/golden/ref_random_golden.npz.
 """
+import hashlib
 import os
 
 import numpy as np
-import pytest
 
 from oracle import pyoracle as po
 
@@ -108,26 +108,32 @@ def test_jhash_golden(golden_dir):
     assert [L.gyo_jhash2(po._p(words), n, 0xceedfead) for n in range(13)] == g["hwords"].tolist()
 
 
-# ---- 3. live against the compiled reference ------------------------------------------------------------
-@pytest.mark.skipif(po.ref() is None, reason="oracle/_ref/libgyref.so not built (no reference tree)")
-def test_oracle_vs_compiled_reference_random():
-    R = po.ref()
-    assert R.gyref_sizeof_hist_resp() == 280
+# ---- 3. against the compiled reference on random streams ----------------------------------------------------
+def test_oracle_vs_compiled_reference_random(golden_dir):
+    g = np.load(os.path.join(golden_dir, "ref_random_golden.npz"))
+    assert g["sizeof_hist_resp"][0] == 280
     rng = np.random.default_rng(7)
-    pcts = [25, 50, 95, 99, 99.9]
+    pcts = g["pcts"].tolist()
+    i = 0
     for name, cls in po.CLS.items():
         if name.startswith("FD_"):
             continue
         for tk in (po.T_INT64, po.T_INT):
             for scale in (50, 5000, 2 ** 20, 2 ** 34):
                 vals = rng.integers(-scale // 10, scale, 5000, dtype=np.int64)
+                assert g["case"][i].tolist() == [cls, tk, scale]
+                assert hashlib.sha256(vals.tobytes()).digest() == g["vals_sha256"][i].tobytes(), "not the stream the reference saw"
                 a = run(cls, tk, vals, pcts)
-                b = po.hist_run(R, "gyref_hist_run", cls, tk, vals, pcts)
+                nb = int(g["nb"][i])
                 for k in ("nb", "total", "max"):
-                    assert a[k] == b[k], (name, tk, scale, k)
-                assert np.array_equal(a["buckets"], b["buckets"]), (name, tk, scale)
-                assert np.array_equal(a["stats"], b["stats"]), (name, tk, scale)
-                assert np.array_equal(a["pct"], b["pct"]), (name, tk, scale)
-                assert np.float32(a["avg"]) == np.float32(b["avg"])
+                    assert a[k] == g[k][i], (name, tk, scale, k)
+                assert np.array_equal(a["buckets"], g["buckets"][i]), (name, tk, scale)
+                assert np.array_equal(a["stats"]["count"], g["count"][i][:nb]), (name, tk, scale)
+                assert np.array_equal(a["stats"]["sum"], g["sum"][i][:nb]), (name, tk, scale)
+                assert np.array_equal(a["pct"], g["pct"][i]), (name, tk, scale)
+                assert np.float32(a["avg"]) == g["avg"][i]
+                i += 1
+    assert i == len(g["case"]) == 64
     keys = rng.integers(0, 2 ** 64, 2000, dtype=np.uint64)
-    assert [L.gyo_uint64_hash(int(k)) for k in keys] == [R.gyref_uint64_hash(int(k)) for k in keys]
+    assert np.array_equal(keys, g["keys"])
+    assert [L.gyo_uint64_hash(int(k)) for k in keys] == g["h64"].tolist()
