@@ -82,6 +82,8 @@ def lib():
         L.gyo_td_init.argtypes = [C.c_void_p]
         L.gyo_td_add_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_double]
         L.gyo_td_add_classic.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_double]
+        L.gyo_td_compress.restype = C.c_uint32
+        L.gyo_td_compress.argtypes = [C.c_void_p, C.c_uint32, C.c_double, C.c_void_p, C.c_uint32]
         L.gyo_td_quantile.restype = C.c_double
         L.gyo_td_quantile.argtypes = [C.c_void_p, C.c_uint32, C.c_double, C.c_double, C.c_double]
         L.gyo_td_quantile_f.restype = C.c_double
@@ -266,6 +268,27 @@ class OracleEngine:
 
 def td_quantile(td, q):
     return lib().gyo_td_quantile(C.byref(td), td.n, td.minv, td.maxv, q)
+
+
+def td_compress(means, weights, delta):
+    """gyo_td_compress of one mean-sorted centroid list -> (means, weights) of at most TD_CAP clusters"""
+    src = np.zeros(len(means), dtype=CENTROID_DTYPE)
+    src["mean"], src["weight"] = means, weights
+    out = np.zeros(TD_CAP, dtype=CENTROID_DTYPE)
+    n = lib().gyo_td_compress(_p(src), len(src), float(delta), _p(out), TD_CAP)
+    assert n <= TD_CAP, n
+    return out["mean"][:n].copy(), out["weight"][:n].copy()
+
+
+def merge_compress(a, b, delta):
+    """what the merge kernels do with two digests a, b = (means, weights): a stable merge by mean, `a` first on equal means, then
+    the fixed-grid compress. Both lists are sorted by mean, so a stable sort of a + b is that merge."""
+    means = np.concatenate([np.asarray(a[0], dtype=np.float64), np.asarray(b[0], dtype=np.float64)])
+    weights = np.concatenate([np.asarray(a[1], dtype=np.uint64), np.asarray(b[1], dtype=np.uint64)])
+    if not len(means):
+        return means, weights
+    order = np.argsort(means, kind="stable")
+    return td_compress(means[order], weights[order], delta)
 
 
 def td_new():

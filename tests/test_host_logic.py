@@ -127,6 +127,34 @@ def test_oracle_engine_sharded_merge_equals_single():
         assert np.array_equal(merged.export_hll(int(id_)), one.export_hll(int(id_)))
 
 
+@pytest.mark.parametrize("delta", [10, 37, 200, 256])
+def test_merge_compress_equals_the_oracle_merge(delta):
+    """pyoracle.merge_compress (the CPU replay of the merge kernels' digest fold) gives the same centroids, bit for bit, as the
+    digest merge of gyo_merge_from, which walks the merged list in C"""
+    rng = np.random.default_rng(12)
+    ev = synth.gen_mixed(rng, 40_000, 60, ntask=8, nhosts=16, nclients=2000)
+    ev["host_idx"] = rng.integers(0, 16, len(ev))           # every service on both shards
+    sh = [po.OracleEngine(max_svcs=128, max_tasks=16, cms_log2_width=8, td_compression=delta, rank=r, world=2) for r in range(2)]
+    for s in sh:
+        for off in range(0, len(ev), 4096):
+            s.ingest(ev[off: off + 4096])
+    merged = po.OracleEngine(max_svcs=128, max_tasks=16, cms_log2_width=8, td_compression=delta)
+    merged.merge_from(sh[0]); merged.merge_from(sh[1])
+    nboth = 0
+    for id_ in np.unique(ev["svc_id"][ev["type"] == 5]):
+        parts = [s.export_tdigest(int(id_)) for s in sh]
+        acc = (np.zeros(0), np.zeros(0, dtype=np.uint64))
+        for td in parts:
+            if td is not None:
+                acc = po.merge_compress(acc, td.centroids(), delta)
+        nboth += all(td is not None and td.n for td in parts)
+        m, w = merged.export_tdigest(int(id_)).centroids()
+        assert np.array_equal(acc[0], m) and np.array_equal(acc[1], w), hex(int(id_))
+        assert len(m) <= delta
+    assert nboth >= 10
+    assert po.merge_compress(([], []), ([], []), delta)[0].size == 0
+
+
 def test_oracle_idle_eviction_rule():
     """the checker's own statement of the listener deletion rule (common/gy_socket_stat.cc:3968-3982): never-active services
     stay (tclock == 0), an idle one goes only when last activity + 300 s < now AND first seen + 600 s < now, its slot is
